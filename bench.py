@@ -43,6 +43,7 @@ import sys
 import tempfile
 import threading
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -267,6 +268,36 @@ def timed_loop(step_fn, steps, device, world, sampler=None):
     return _max_over_ranks(total, device, world), statistics.median(gaps), host_ms, gaps
 
 
+# Per-array caps of --dump-outputs: 2 outputs x 16 MiB + 186 parameters x 128 KiB < 64 MiB
+DUMP_OUTPUT_ELEMS, DUMP_GRAD_ELEMS, DUMP_MAX_BYTES = 1 << 22, 1 << 15, 64 << 20
+
+
+def _dump_array(t, cap, name):
+    """float32 host copy of `t`; above `cap` elements, the same `cap` positions (drawn from a
+    generator seeded with the name) of the flattened tensor in every run and build."""
+    t = t.detach()
+    if t.numel() > cap:
+        g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+        idx = torch.randint(t.numel(), (cap,), generator=g).sort().values
+        t = t.flatten()[idx.to(t.device)]
+    return t.float().cpu().numpy()
+
+
+def dump_outputs(out_dir, outputs, model):
+    """What one timed step hands its caller: the clip outputs (`clip.npy`), the query rows
+    (`query.npy`) and every parameter's gradient (`grad.<parameter name>.npy`), float32."""
+    import numpy as np
+    arrays = {k: _dump_array(v, DUMP_OUTPUT_ELEMS, k) for k, v in outputs.items()}
+    for name, p in model.named_parameters():
+        if p.grad is not None:
+            arrays["grad." + name] = _dump_array(p.grad, DUMP_GRAD_ELEMS, name)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_ours(args):
     from hero_b200 import distributed as hdist
     from hero_b200 import ops, synth
@@ -333,7 +364,7 @@ def run_ours(args):
             if clip_norm is not None:
                 opt.clip_grad_norm_device_(clip_norm)
             opt.step()
-        return clip
+        return clip, q
 
     # ------------------------------------------------------------- device-resident timing
     resident = []
@@ -342,12 +373,15 @@ def run_ours(args):
         qb = attach_plan(dict(qb), kind="txt")
         resident.append((synth.to_device(vb, device), synth.to_device(qb, device)))
     torch.cuda.synchronize()
+    last = {}     # outputs of the latest resident step, kept only for --dump-outputs
 
     def resident_step(i):
         if state["micro"] % state["accum"] == 0:
             (flat.zero_grads_async() if args.grad_zero == "async" else gflat.zero_())
         vb_dev, qb_dev = resident[i % n_host]
-        fwd_bwd(vb_dev, qb_dev)
+        clip, q = fwd_bwd(vb_dev, qb_dev)
+        if args.dump_outputs:
+            last["clip"], last["query"] = clip.detach(), q.detach()
 
     # known-answer test of the gradient exchange on this job's ranks / transport (raises on a
     # mismatch): every rank must end with the mean of the per-rank patterns, bit-identical
@@ -373,6 +407,8 @@ def run_ours(args):
         time.sleep(0.2)
     ms_total, ms_median, host_enqueue_ms, gaps = timed_loop(resident_step, args.steps, device,
                                                             world, sampler)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, model)
     host_free_ms = round(statistics.median(HOST_FREE_MS), 3) if HOST_FREE_MS else None
     launches = ops.launch_count() // max(args.steps, 1)
     ms_per_step = ms_total / args.steps
@@ -560,7 +596,7 @@ def run_ours(args):
             if state["micro"] % accum == 0:
                 (flat.zero_grads_async() if args.grad_zero == "async" else gflat.zero_())
             t_b = time.perf_counter()
-            clip = fwd_bwd(vb_dev, qb_dev)
+            clip, _ = fwd_bwd(vb_dev, qb_dev)
             t_c = time.perf_counter()
             slot = result_host[i % (RESULT_LAG + 1):i % (RESULT_LAG + 1) + 1]
             # (detach: the pinned result buffer must not become part of — and keep alive — the
@@ -901,6 +937,10 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-clips", type=int, default=8)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's outputs and parameter gradients "
+                         "of the last timed step as DIR/<name>.npy (float32; arrays above a size "
+                         "cap as a fixed seeded sample) to compare builds on identical inputs")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -3,7 +3,8 @@
 imports point at hero_b200 — (A) keeping the reference's HierarchicalVlModel / HeroModel classes
 over hero_b200's CrossModalTrm / TemporalTrm / LinearLayer, (B) also re-exporting hero_b200's
 packed-path classes — and reproduce the goldens of the unmodified reference. Needs the reference
-sources (/root/reference in the build container, or the staged baseline/_ref): skipped elsewhere."""
+sources (a checkout named by HERO_REFERENCE, or the copy baseline/stage_ref.py staged under
+baseline/_ref): skipped elsewhere."""
 import json
 import os
 import subprocess
@@ -15,9 +16,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _reference_dir():
-    for cand in (os.environ.get("HERO_REFERENCE", "/root/reference"),
-                 os.path.join(ROOT, "baseline", "_ref")):
-        if os.path.isfile(os.path.join(cand, "model", "model.py")):
+    for cand in (os.environ.get("HERO_REFERENCE"), os.path.join(ROOT, "baseline", "_ref")):
+        if cand and os.path.isfile(os.path.join(cand, "model", "model.py")):
             return cand
     return None
 
