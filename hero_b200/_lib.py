@@ -97,8 +97,6 @@ class StackArgs(C.Structure):
         ("drop_key", C.c_uint32),
         ("hidden_drop_scale", C.c_float), ("attn_drop_scale", C.c_float),
         ("dout", C.c_void_p), ("dx", C.c_void_p), ("scratch", C.c_void_p),
-        ("first_layer", C.c_int32),
-        ("layer_done_events", C.POINTER(C.c_void_p)),
     ]
 
 
@@ -108,8 +106,6 @@ def _declare(lib):
     lib.hero_last_error.argtypes = []
     lib.hero_version.restype = C.c_int
     lib.hero_sm_count.restype = C.c_int
-    lib.hero_set_sm_limit.restype = C.c_int
-    lib.hero_set_sm_limit.argtypes = [i32]
     lib.hero_gemm_bf16.restype = C.c_int
     lib.hero_gemm_bf16.argtypes = [C.POINTER(GemmArgs), vp]
 
@@ -141,7 +137,6 @@ def _declare(lib):
     sig("hero_adamw_step", vp, vp, vp, vp, vp, i64, f32, f32, f32, f32, f32, f32, vp, f32, vp)
     sig("hero_sumsq_f32", vp, i64, vp, vp)
     sig("hero_ce_finish", vp, i64, i32, vp, i32, vp, vp, vp)
-    sig("hero_reduce_slots_f32", vp, vp, i32, i64, i64, f32, i32, vp)
     sig("hero_l2norm_split_f32", vp, i64, i32, f32, vp, vp, vp, vp)
     sig("hero_vsm_masked_max", vp, i64, vp, i32, i32, i32, vp, vp, vp)
     sig("hero_vsm_scores_bwd", vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp)

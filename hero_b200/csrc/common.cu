@@ -28,17 +28,15 @@ bool serial_profiling() {
   return on;
 }
 
-static int g_sm_limit = 0;
-
 int sm_count() {
   static int cached = 0;
-  if (cached > 0) return (g_sm_limit > 0 && g_sm_limit < cached) ? g_sm_limit : cached;
+  if (cached > 0) return cached;
   int dev = 0, n = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return -HERO_ERR_NO_DEVICE;
   if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
     return -HERO_ERR_NO_DEVICE;
   cached = n;
-  return (g_sm_limit > 0 && g_sm_limit < cached) ? g_sm_limit : cached;
+  return cached;
 }
 
 int encode_tmap_2d_bf16(void* map, const void* ptr, long long inner, long long outer, long long ld,
@@ -82,8 +80,3 @@ int hero_sm_count(void) {
 }
 
 }  // extern "C"
-
-extern "C" int hero_set_sm_limit(int32_t n) {
-  hero::g_sm_limit = n > 0 ? n : 0;
-  return HERO_OK;
-}

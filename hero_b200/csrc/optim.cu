@@ -105,40 +105,9 @@ ce_finish_kernel(const float2* __restrict__ part, long long ld, int n_slabs,
   loss[r] = l - lab[r];
 }
 
-// dst[i] = (dst[i] + sum_s slots[s * stride + i]) * scale: the reduction step of the copy-engine
-// gradient exchange (peers have written their contributions into `slots`).
-__global__ void reduce_slots_kernel(float* __restrict__ dst, const float* __restrict__ slots,
-                                    int n_slots, long long stride, long long n4, float scale) {
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
-       i += (long long)gridDim.x * blockDim.x) {
-    float4 acc = reinterpret_cast<const float4*>(dst)[i];
-    for (int s = 0; s < n_slots; ++s) {
-      const float4 v = reinterpret_cast<const float4*>(slots + s * stride)[i];
-      acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-    }
-    acc.x *= scale; acc.y *= scale; acc.z *= scale; acc.w *= scale;
-    reinterpret_cast<float4*>(dst)[i] = acc;
-  }
-}
-
 }  // namespace hero
 
 using namespace hero;
-
-extern "C" int hero_reduce_slots_f32(float* dst, const float* slots, int32_t n_slots,
-                                     int64_t slot_stride, int64_t n, float scale,
-                                     int32_t max_ctas, void* stream) {
-  HERO_REQUIRE(dst && (slots || n_slots == 0) && n >= 0 && n % 4 == 0 && slot_stride % 4 == 0,
-               "reduce_slots: bad args (n and stride must be multiples of 4)");
-  if (n == 0) return HERO_OK;
-  long long blocks = (n / 4 + 255) / 256;
-  const long long cap = max_ctas > 0 ? max_ctas : 64;
-  if (blocks > cap) blocks = cap;
-  reduce_slots_kernel<<<(unsigned)blocks, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-      dst, slots, n_slots, slot_stride, n / 4, scale);
-  HERO_LAUNCH_CHECK();
-  return HERO_OK;
-}
 
 extern "C" int hero_adamw_step(float* p, const float* g, float* m, float* v, void* p_bf16,
                                int64_t n, float step_size, float beta1, float beta2, float eps,

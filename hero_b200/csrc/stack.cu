@@ -155,11 +155,11 @@ extern "C" int hero_bert_stack_fwd(const hero_stack_args* s, void* stream) {
     HERO_STEP(ABL_ATTN_FWD, hero_attn_fwd(A.qkv, s->tile_tok0, s->tile_ntok, s->seq_lo, s->seq_hi, A.cx, A.lse, M,
                            s->n_tiles, s->n_long, s->max_long, s->heads, 64, scale,
                            s->attn_drop_threshold,
-                           site_key(s->drop_key, s->first_layer + l, 0), s->attn_drop_scale, stream));
+                           site_key(s->drop_key, l, 0), s->attn_drop_scale, stream));
     // residual of the attention block = this layer's input in fp32: the caller's fp32 copy for
     // layer 0, LayerNorm(previous layer's s2) recomputed in the epilogue afterwards
     Gemm outp(A.cx, H, 0, W.wo, H, 0, M, H, H, A.s1, H);
-    outp.bias(W.bo).drop(s->hidden_drop_threshold, site_key(s->drop_key, s->first_layer + l, 1),
+    outp.bias(W.bo).drop(s->hidden_drop_threshold, site_key(s->drop_key, l, 1),
                          s->hidden_drop_scale);
     if (l == 0) {
       outp.resid_f32(s->x_f32, H);
@@ -180,7 +180,7 @@ extern "C" int hero_bert_stack_fwd(const hero_stack_args* s, void* stream) {
     HERO_STEP(ABL_FWD_GEMM, Gemm(A.f, I, 0, W.w2, I, 0, M, H, I, A.s2, H)
                  .bias(W.b2)
                  .resid_ln(A.s1, H, A.mean1, A.rstd1, W.ln1_g, W.ln1_b)
-                 .drop(s->hidden_drop_threshold, site_key(s->drop_key, s->first_layer + l, 2), s->hidden_drop_scale)
+                 .drop(s->hidden_drop_threshold, site_key(s->drop_key, l, 2), s->hidden_drop_scale)
                  .run(stream));
     ln_base(&ln, A.s2, W.ln2_g, W.ln2_b, s->eps, M, H, A.mean2, A.rstd2);
     ln.y = A.out;
@@ -256,7 +256,7 @@ extern "C" int hero_bert_stack_bwd(const hero_stack_args* s, void* stream) {
     if (hd) {
       ln.dx_drop = ds2_d;
       ln.drop2_threshold = s->hidden_drop_threshold;
-      ln.drop2_key = site_key(s->drop_key, s->first_layer + l, 2);
+      ln.drop2_key = site_key(s->drop_key, l, 2);
       ln.drop2_scale = s->hidden_drop_scale;
       g2 = ds2_d;
     }
@@ -278,7 +278,7 @@ extern "C" int hero_bert_stack_bwd(const hero_stack_args* s, void* stream) {
     if (hd) {
       ln.dx_drop = ds1_d;
       ln.drop2_threshold = s->hidden_drop_threshold;
-      ln.drop2_key = site_key(s->drop_key, s->first_layer + l, 1);
+      ln.drop2_key = site_key(s->drop_key, l, 1);
       ln.drop2_scale = s->hidden_drop_scale;
       g1 = ds1_d;
     }
@@ -291,7 +291,7 @@ extern "C" int hero_bert_stack_bwd(const hero_stack_args* s, void* stream) {
     HERO_STEP(ABL_ATTN_BWD, hero_attn_bwd(A.qkv, s->tile_tok0, s->tile_ntok, s->seq_lo, s->seq_hi, A.cx, dcx, A.lse,
                            dqkv, G.dbqkv, M, s->n_tiles, s->n_long, s->max_long, s->heads, 64, scale,
                            s->attn_drop_threshold,
-                           site_key(s->drop_key, s->first_layer + l, 0), s->attn_drop_scale, stream));
+                           site_key(s->drop_key, l, 0), s->attn_drop_scale, stream));
     HERO_TRY(publish());
     // QKV projection
     HERO_STEP(ABL_WGRAD, Gemm(dqkv, 3 * H, 1, h_in, H, 1, 3 * H, H, M, G.dwqkv, H).f32_accumulate().run(wstream));
@@ -299,11 +299,6 @@ extern "C" int hero_bert_stack_bwd(const hero_stack_args* s, void* stream) {
       HERO_CUDA_CHECK(cudaEventRecord(side->done[par], side->stream));
       done_recorded[par] = true;
     }
-    // every parameter gradient of layer l is complete here: the side stream has waited for the
-    // chain's LayerNorm / attention kernels (publish) and has just issued the last weight gradient
-    if (s->layer_done_events != nullptr && s->layer_done_events[l] != nullptr)
-      HERO_CUDA_CHECK(cudaEventRecord(reinterpret_cast<cudaEvent_t>(s->layer_done_events[l]),
-                                      two_streams ? side->stream : chain));
     void* dx = (l == 0 && s->dx) ? s->dx : ((l & 1) ? dxa : dxb);
     if (l > 0 || s->dx)
       HERO_STEP(ABL_DGRAD, Gemm(dqkv, 3 * H, 0, W.wqkv, H, 1, M, H, 3 * H, dx, H).resid(ds1, H).run(stream));

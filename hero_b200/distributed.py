@@ -16,7 +16,6 @@ torchrun-style environment variables.
 """
 import os
 import pickle
-import sys
 
 import torch
 import torch.distributed as dist
@@ -268,338 +267,26 @@ def any_broadcast(data, root_rank):
     return box[0]
 
 
-def bucket_parts(a, b, world, align=64):
-    """Split the flat range [a, b) into `world` consecutive parts of `chunk` elements (a multiple of
-    `align`; the last parts may be short or empty). Returns (parts, chunk)."""
-    n = b - a
-    chunk = (-(-n // world) + align - 1) // align * align
-    parts = [(min(a + r * chunk, b), min(a + (r + 1) * chunk, b)) for r in range(world)]
-    return parts, chunk
-
-
-class PeerExchange:
-    """Mean all-reduce of ranges of the flat gradient buffer with DMA copies over NVLink instead of
-    a communication kernel (the buckets that travel while backward is still running).
-
-    The gradient buffer and a staging buffer live in symmetric memory
-    (torch.distributed._symmetric_memory: every rank maps every peer's allocation). For a bucket
-    [a, b) split into `world` parts, rank r owns part r:
-      1. reduce-scatter: every rank copies its values of part r into a staging slot on rank r
-         (cudaMemcpyAsync to the peer mapping = copy engines, no SMs) and signals r;
-      2. rank r adds the world-1 slots to its own values and scales by 1/world
-         (`hero_reduce_slots_f32`, the only kernel: <= 16 CTAs, HBM-bound);
-      3. all-gather: rank r copies the reduced part into every peer's gradient buffer and signals.
-    Everything is enqueued on one side stream, ordered after the event that marks the bucket
-    final. NCCL kernels cannot do this job beside the GEMMs: the GEMMs run one CTA per SM, a
-    full-speed NCCL kernel wants ~24 SMs, a 4-8 CTA one moves 90-170 GB/s and was measured to finish
-    only after backward (tools/dp_timeline.py, tools/allreduce_probe.py)."""
-
-    def __init__(self, flat, group=None):
-        import torch.distributed._symmetric_memory as symm
-        group = dist.group.WORLD if group is None else group
-        self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
-        dev = flat.flat.device
-        try:
-            symm.enable_symm_mem_for_group(group.group_name)
-        except Exception:       # newer torch enables every group implicitly
-            pass
-        pad = 64 * self.world
-        self.grad = symm.empty(flat.total + pad, dtype=torch.float32, device=dev)
-        self.stage = symm.empty(flat.total + pad, dtype=torch.float32, device=dev)
-        self.h_grad = symm.rendezvous(self.grad, group.group_name)
-        self.h_stage = symm.rendezvous(self.stage, group.group_name)
-        self.grad.zero_()
-        self.stream = torch.cuda.Stream(dev, priority=-1)
-        self.channels = max(1, min(128, self.h_grad.signal_pad_size // (4 * self.world) - 1))
-        self.flat = flat
-        flat.adopt_grad_buffer(self.grad)
-        torch.cuda.synchronize(dev)
-        self.h_grad.barrier(0)
-
-    def fits(self, a, b):
-        _, chunk = bucket_parts(a, b, self.world)
-        return (self.world - 1) * chunk <= b - a      # staging of a bucket stays inside [a, b)
-
-    def exchange(self, a, b, event=None, reduce_ctas=16):
-        """Enqueue the exchange of [a, b) behind `event` (default: behind everything already on
-        the current stream). `reduce_ctas` caps the reduction kernel (small beside backward)."""
-        if event is None:
-            event = torch.cuda.Event()
-            event.record()
-        self.stream.wait_event(event)
-        with torch.cuda.stream(self.stream):
-            self._scatter(a, b)
-            self._reduce(a, b, reduce_ctas)
-            self._gather(a, b)
-
-    def _others(self):
-        return [(self.rank + k) % self.world for k in range(1, self.world)]
-
-    def _plan(self, a, b):
-        """Views and peer mappings of a bucket (the same buckets recur every step: cached)."""
-        plans = self.__dict__.setdefault("_plans", {})
-        pl = plans.get((a, b))
-        if pl is None:
-            W, me = self.world, self.rank
-            parts, chunk = bucket_parts(a, b, W)
-            lo, hi = parts[me]
-            # one signal channel per bucket (pads hold >= 128 channels): a bucket's signals never
-            # queue behind another bucket's, and the "gathered" acknowledgements can all be
-            # collected at the end of the step instead of stalling the stream after every bucket
-            pl = {"chunk": chunk, "lo": lo, "hi": hi, "scatter": [], "gather": [],
-                  "channel": len(plans) % self.channels,
-                  "wait_gather": [p for p in self._others() if parts[p][1] > parts[p][0]]}
-            for r in self._others():
-                rlo, rhi = parts[r]
-                if rhi > rlo:
-                    slot = (me - r - 1) % W        # 0 .. W-2: which of r's slots is mine
-                    dst = self.h_stage.get_buffer(r, (rhi - rlo,), torch.float32,
-                                                  a + slot * chunk)
-                    pl["scatter"].append((r, dst, self.grad[rlo:rhi]))
-                if hi > lo:
-                    dst = self.h_grad.get_buffer(r, (hi - lo,), torch.float32, lo)
-                    pl["gather"].append((r, dst))
-            if hi > lo:
-                assert (hi - lo) % 4 == 0 and lo % 4 == 0   # FlatParams aligns everything to 64
-                pl["mine"] = self.grad[lo:hi]
-                pl["slots"] = self.stage[a:]
-            plans[(a, b)] = pl
-        return pl
-
-    def _scatter(self, a, b):
-        """1. my values of part r -> r's staging slot for me, then tell r."""
-        pl = self._plan(a, b)
-        for r, dst, src in pl["scatter"]:
-            dst.copy_(src, non_blocking=True)
-            self.h_stage.put_signal(r, pl["channel"])
-
-    def _reduce(self, a, b, reduce_ctas=16):
-        """2. once every peer's slice of my part has arrived: mean into my gradients."""
-        from . import ops
-        pl = self._plan(a, b)
-        if pl["hi"] > pl["lo"]:
-            for p in self._others():
-                self.h_stage.wait_signal(p, pl["channel"])
-            ops.reduce_slots(pl["mine"], pl["slots"], self.world - 1, pl["chunk"],
-                             1.0 / self.world, max_ctas=reduce_ctas)
-
-    def _gather(self, a, b):
-        """3. my reduced part -> every peer's gradient buffer; wait for theirs."""
-        pl = self._plan(a, b)
-        for r, dst in pl["gather"]:
-            dst.copy_(pl["mine"], non_blocking=True)
-            self.h_grad.put_signal(r, pl["channel"])
-        self.__dict__.setdefault("_unacked", []).append(pl)
-
-    def join(self):
-        """Collect the peers' "gathered" signals of every bucket of the step, then make the current
-        stream wait for every exchange enqueued so far."""
-        with torch.cuda.stream(self.stream):
-            for pl in self.__dict__.pop("_unacked", []):
-                for p in pl["wait_gather"]:
-                    self.h_grad.wait_signal(p, pl["channel"])
-        ev = torch.cuda.Event()
-        ev.record(self.stream)
-        torch.cuda.current_stream().wait_event(ev)
-
-
-class GradBucketer:
-    """Overlaps the data-parallel gradient exchange with the rest of the backward pass.
-
-    The reference all-reduces one flat copy of every gradient AFTER backward has finished
-    (utils/distributed.py:19-46, called at train_vcmr.py:233-239). Here gradients are accumulated
-    in place in FlatParams' flat fp32 buffer, and the hand-written transformer backward reports
-    each layer's parameters as soon as their gradient is final: the ranges of the flat buffer they
-    cover are all-reduced (mean) right away on the communicator's stream while the layers below
-    are still being differentiated. `finish()` reduces every range not covered so far and waits.
-    The result equals one all_reduce_flat(grad_flat) after backward.
-
-    Usage (one step):
-        with bucketer:                 # installs the hook for forward + backward
-            loss = model(...); loss.backward()
-        bucketer.finish(); optimizer.step()
-
-    A parameter used by several forward calls (e.g. c_encoder for video rows and again for query
-    rows) is exchanged only after its LAST backward: forward registers every use (`expect`),
-    backward retires them (`ready`)."""
-
-    def __init__(self, flat, min_elems=1 << 20, overlap_ctas=0, transport="auto"):
-        """transport: how buckets travel while backward is running —
-        "p2p" (PeerExchange: symmetric memory + copy engines, NCCL backend only), "nccl"
-        (an extra communicator capped at `overlap_ctas` CTAs, with the compute kernels sized for
-        that many fewer SMs), "auto" = p2p when available else the default communicator.
-        The remainder after backward always goes through the default, full-speed communicator."""
-        self.flat = flat
-        self.min_elems = min_elems       # merge announced ranges into messages of >= 4 MB
-        self.overlap_ctas = overlap_ctas
-        self.pg = None
-        self.p2p = None
-        self.p2p_tail_max_world = 0
-        nccl = size() > 1 and dist.get_backend() == "nccl"
-        if nccl and transport in ("auto", "p2p"):
-            try:
-                self.p2p = PeerExchange(flat)
-            except Exception as e:          # no symmetric memory on this system
-                if transport == "p2p":
-                    raise
-                import warnings
-                warnings.warn(f"GradBucketer: peer exchange unavailable ({e!r}); using NCCL")
-        if nccl and self.p2p is None and overlap_ctas > 0:
-            opts = dist.ProcessGroupNCCL.Options()
-            opts.config.max_ctas = overlap_ctas
-            opts.config.min_ctas = 1
-            # its CTAs must win the SMs the compute kernels leave free as soon as they are free:
-            # without priority the exchange kernel sat behind the thousands of queued attention /
-            # LayerNorm CTAs and only ran after backward had finished (tools/dp_timeline.py)
-            opts.is_high_priority_stream = True
-            self.pg = dist.new_group(backend="nccl", pg_options=opts)
-        self.reset()
-
-    def reset(self):
-        self.pending = {}       # id(param) -> forward uses whose backward has not run yet
-        self.done = []          # [a, b) ranges of the flat buffer already handed to the backend
-        self.handles = []
-        self.queue = []         # final but not yet sent ranges (waiting to reach min_elems)
-
-    # ---- hook protocol (hero_b200.functional.GRAD_HOOK) -------------------------------------
-    def expect(self, params):
-        for p in params:
-            self.pending[id(p)] = self.pending.get(id(p), 0) + 1
-
-    wants_events = True      # the stack backward stays one native call (functional.py)
-
-    def ready(self, params, event=None):
-        """`event`: CUDA event after which the gradients of `params` are complete (else: complete
-        in current-stream order at the time of the call)."""
-        gf = self.flat.grad_flat
-        if gf is None or size() == 1:
-            return
-        base, spans = gf.data_ptr(), []
-        for p in params:
-            k = id(p)
-            left = self.pending.get(k, 1) - 1
-            self.pending[k] = left
-            ent = self.flat._by_id.get(k)
-            if left > 0 or ent is None or p.grad is None:
-                continue
-            if p.grad.data_ptr() != base + 4 * ent[0]:
-                continue                # gradient does not live in the flat buffer: finish() only
-            spans.append(ent)
-        for off, n in sorted(spans):
-            end = min((off + n + 63) // 64 * 64, self.flat.total)   # alignment padding is zeros
-            if self.queue and off <= self.queue[-1][1]:
-                self.queue[-1][1] = max(self.queue[-1][1], end)
-            else:
-                self.queue.append([off, end])
-        if sum(b - a for a, b in self.queue) >= self.min_elems:
-            self._flush(event)
-
-    def __enter__(self):
-        from . import functional, ops
-        self.reset()
-        functional.GRAD_HOOK[0] = self
-        if self.pg is not None:
-            ops.set_sm_limit(0)
-            ops.set_sm_limit(max(ops.sm_count() - self.overlap_ctas, 1))
-        return self
-
-    def __exit__(self, *exc):
-        from . import functional, ops
-        functional.GRAD_HOOK[0] = None
-        if self.pg is not None:
-            ops.set_sm_limit(0)
-        return False
-
-    # ---- exchange ------------------------------------------------------------------------------
-    def _launch(self, a, b, group=None):
-        if b <= a:
-            return
-        buf = self.flat.grad_flat[a:b]
-        if dist.get_backend() == "nccl":
-            self.handles.append((dist.all_reduce(buf, op=dist.ReduceOp.AVG, group=group,
-                                                 async_op=True), None))
-        else:
-            self.handles.append((dist.all_reduce(buf, op=dist.ReduceOp.SUM, async_op=True), buf))
-        self.done.append((a, b))
-
-    def _flush(self, event=None):
-        for a, b in self.queue:
-            if self.p2p is not None and self.p2p.fits(a, b):
-                self.p2p.exchange(a, b, event)   # beside the backward: copy engines
-                self.done.append((a, b))
-            else:
-                if event is not None:            # NCCL orders itself after the current stream
-                    torch.cuda.current_stream().wait_event(event)
-                self._launch(a, b, self.pg)      # (capped) communicator
-        self.queue = []
-
-    def finish(self, rescale_denom=1.0):
-        """Exchange every range not sent so far, wait for all of it (the current stream waits; the
-        host does not block on NCCL) and apply the reference's rescale."""
-        timing = os.environ.get("HERO_DP_TIMING") == "1"
-        marks = []
-
-        def mark(name):
-            if timing:
-                e = torch.cuda.Event(enable_timing=True)
-                e.record()
-                marks.append((name, e))
-
-        if size() > 1:
-            self.flat.ensure_flat_grads()
-            mark("backward enqueued work done")
-            rest = [tuple(r) for r in self.queue]
-            self.queue = []
-            pos = 0
-            for a, b in sorted(self.done):
-                if a > pos:
-                    rest.append((pos, a))
-                pos = max(pos, b)
-            if pos < self.flat.total:
-                rest.append((pos, self.flat.total))
-            # After backward nothing competes for SMs: the remainder goes through the full-speed
-            # NCCL communicator (176 MB in 0.5-0.6 ms at N = 2; the peer-copy path was measured at
-            # 0.7-0.8 ms for the same bytes - `p2p_tail_max_world` > 0 re-enables it for A/B runs).
-            for a, b in rest:
-                if self.p2p is not None and size() <= self.p2p_tail_max_world and self.p2p.fits(a, b):
-                    self.p2p.exchange(a, b, reduce_ctas=592)
-                else:
-                    self._launch(a, b)
-            n_tail = len(self.handles)
-            for h, buf in self.handles:
-                h.wait()
-                if buf is not None:
-                    buf.div_(size())
-            mark(f"remainder through NCCL ({n_tail} calls)")
-            if self.p2p is not None:
-                self.p2p.join()
-                mark("peer exchanges joined")
-        if rescale_denom != 1.0:
-            self.flat.grad_flat.div_(rescale_denom)
-        if timing and marks:
-            torch.cuda.synchronize()
-            print("GradBucketer.finish device ms:",
-                  [(b[0], round(a[1].elapsed_time(b[1]), 3)) for a, b in zip(marks[:-1], marks[1:])],
-                  file=sys.stderr)
-        self.reset()
-
-
 def overlapped_exchange(flat, transport="none", **kw):
-    """The gradient-exchange schedule for a training loop: None = one NCCL all-reduce of the flat
-    buffer after backward (`all_reduce_flat`, the reference's schedule — the default), or a
-    GradBucketer ("p2p": buckets travel as peer copies during backward, "nccl": through a capped
-    communicator).
+    """The gradient-exchange schedule selected by a training loop's `transport` option. Only
+    None / "none" remains: the caller exchanges the gradients with FlatGradExchange (or
+    `all_reduce_flat`) after or beside backward, and None is returned. Other keyword arguments
+    (options of the removed schedule below) are ignored.
 
+    A bucketed schedule that sent per-layer buckets during backward ("p2p": peer copies over
+    symmetric memory, "nccl": a communicator capped in CTAs) was removed after losing to it on
     B200 / NVSwitch, 430 MB of fp32 gradients, 6.4-6.5 ms of compute per step, ms per step:
-      N = 2: bucketer 7.23-7.34 device-resident but 7.96 end to end (its ~100 extra host-side
+      N = 2: bucketed 7.23-7.34 device-resident but 7.96 end to end (its ~100 extra host-side
              enqueues per step double the host time of a step), all-reduce after backward 7.32;
-      N = 4: bucketer 8.23, all-reduce after backward 7.65 - every bucket costs 2 (N-1) copies and
+      N = 4: bucketed 8.23, all-reduce after backward 7.65 - every bucket costs 2 (N-1) copies and
              signals per rank, and NCCL's all-reduce grows by only 0.3 ms from N = 2 to N = 4.
-    The bucketer hides its exchanges completely (HERO_DP_TIMING=1) but the 41 % of the bytes that
-    become final only when backward ends stay exposed either way, so it is opt-in."""
-    if size() <= 1 or transport in (None, "none"):
+    It hid its exchanges completely, but the 41 % of the bytes that become final only when
+    backward ends stay exposed either way (DESIGN.md §5)."""
+    if transport in (None, "none"):
         return None
-    return GradBucketer(flat, transport=transport, **kw)
+    raise ValueError(f"gradient exchange transport {transport!r}: the bucketed schedule was "
+                     "removed (measured slower than the default exchange, DESIGN.md §5); "
+                     "use 'none'")
 
 
 class VsmAllgather(torch.autograd.Function):

@@ -19,11 +19,7 @@ BF16 = torch.bfloat16
 F32 = torch.float32
 
 
-# Data-parallel hook (hero_b200.distributed.GradBucketer): forward passes report the parameters
-# they use (`expect`), backward passes report parameters whose gradient contribution is complete
-# (`ready`), so the exchange of a layer's gradients overlaps the backward of the layers below.
-GRAD_HOOK = [None]
-# Lighter protocol of distributed.FlatGradExchange(overlap=True): it counts transformer-stack
+# Data-parallel hook of distributed.FlatGradExchange(overlap=True): it counts transformer-stack
 # forwards / backwards and is told when the cross-modal embedding backward (the last node of the
 # graph) begins — at that point every gradient outside the embedding tables is final and their
 # all-reduce can run beside the embedding backward.
@@ -117,8 +113,6 @@ class _TransformerStack(torch.autograd.Function):
                                                  x_f32=x_f32)
         ctx.cfg, ctx.dspec, ctx.saved, ctx.params = cfg, dspec, saved, params
         ctx.x = x
-        if need_grad and GRAD_HOOK[0] is not None:
-            GRAD_HOOK[0].expect(params)
         if need_grad and EXCHANGE_HOOK[0] is not None:
             EXCHANGE_HOOK[0].stack_forward()
         return out_f32 if cfg.get("out_f32") else out
@@ -128,48 +122,14 @@ class _TransformerStack(torch.autograd.Function):
         cfg, params = ctx.cfg, ctx.params
         if dout.dtype != BF16:
             dout = dout.to(BF16)
-        n = len(cfg["layers"])
         grads, ret = _stack_sinks(cfg, params, ctx.x.shape[1], dout.device)
-        hook = GRAD_HOOK[0]
-        if hook is None:
-            dx = ops.bert_stack_bwd(ctx.x, cfg["layers"], cfg["att"], ctx.saved,
-                                    dout.contiguous(), grads, heads=cfg["heads"], eps=cfg["eps"],
-                                    drop=ctx.dspec, need_dx=ctx.needs_input_grad[0])
-        elif getattr(hook, "wants_events", False) and dout.is_cuda:
-            # data-parallel: ONE native call; the runtime records an event per layer where that
-            # layer's gradients are complete, and the exchanges are enqueued behind those events
-            events = _layer_events(cfg, n, dout.device)
-            dx = ops.bert_stack_bwd(ctx.x, cfg["layers"], cfg["att"], ctx.saved,
-                                    dout.contiguous(), grads, heads=cfg["heads"], eps=cfg["eps"],
-                                    drop=ctx.dspec, need_dx=ctx.needs_input_grad[0],
-                                    layer_events=events)
-            for li in range(n - 1, -1, -1):
-                hook.ready(params[16 * li:16 * li + 16], event=events[li])
-        else:
-            # hooks without event support: one native call per layer
-            dx = dout.contiguous()
-            for li in range(n - 1, -1, -1):
-                dx = ops.bert_stack_bwd(ctx.x, cfg["layers"], cfg["att"], ctx.saved, dx, grads,
-                                        heads=cfg["heads"], eps=cfg["eps"], drop=ctx.dspec,
-                                        need_dx=(li > 0 or ctx.needs_input_grad[0]), only_layer=li)
-                hook.ready(params[16 * li:16 * li + 16])
+        dx = ops.bert_stack_bwd(ctx.x, cfg["layers"], cfg["att"], ctx.saved,
+                                dout.contiguous(), grads, heads=cfg["heads"], eps=cfg["eps"],
+                                drop=ctx.dspec, need_dx=ctx.needs_input_grad[0])
         ctx.saved = None
         if EXCHANGE_HOOK[0] is not None:
             EXCHANGE_HOOK[0].stack_backward()
         return (dx, None, None) + tuple(ret)
-
-
-def _layer_events(cfg, n, device):
-    """n reusable CUDA events for `hero_stack_args.layer_done_events` (kept on the encoder)."""
-    cache = cfg.get("cache")
-    events = None if cache is None else cache.get("events")
-    if events is None or len(events) != n:
-        events = [torch.cuda.Event() for _ in range(n)]
-        for e in events:
-            e.record()            # materialise the cudaEvent_t handle
-        if cache is not None:
-            cache["events"] = events
-    return events
 
 
 def _stack_sinks(cfg, params, H, device):

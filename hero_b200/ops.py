@@ -34,14 +34,8 @@ def launch_count():
 
 
 def sm_count():
-    """SMs the persistent kernels are sized for (the device's count, or the current limit)."""
+    """SMs the persistent kernels are sized for: the device's count."""
     return _lib.lib().hero_sm_count()
-
-
-def set_sm_limit(n):
-    """Size persistent kernels for at most n SMs (0 = all): leaves room for a communication
-    kernel running beside them (`hero_set_sm_limit`)."""
-    _lib.check(_lib.lib().hero_set_sm_limit(int(n)))
 
 
 def start_gemm_profile():
@@ -244,21 +238,6 @@ def attn_bwd(qkv, att, ctx, dctx, lse, dqkv, *, heads, head_dim=64, drop=(0, 0, 
     return dqkv
 
 
-class _PtrTensor:
-    """Minimal stand-in for a tensor that lives inside a workspace (only what _stack_struct
-    reads: data_ptr / shape / device)."""
-
-    def __init__(self, ptr, shape, device):
-        self._ptr, self.shape, self.device = ptr, shape, device
-        self.dtype, self.is_cuda = BF16, True
-
-    def data_ptr(self):
-        return self._ptr
-
-    def is_contiguous(self):
-        return True
-
-
 # kernels launched per layer by the native runtime (for bench.py's gpu_launches)
 _STACK_FWD_LAUNCHES, _STACK_BWD_LAUNCHES = 7, 11   # bwd: 8 GEMM, 2 LN (one pass each), attention
 _ACT_FIELDS = ("qkv", "cx", "lse", "s1", "mean1", "rstd1", "a", "a_f32", "pre", "f", "s2", "mean2",
@@ -356,26 +335,13 @@ def bert_stack_fwd(x, layers, att, *, heads, eps, drop, save, x_f32=None):
     return out, out_f32, ((ws, act_ptrs) if save else None)
 
 
-def bert_stack_bwd(x, layers, att, saved, dout, grads, *, heads, eps, drop, need_dx=True,
-                   only_layer=None, layer_events=None):
+def bert_stack_bwd(x, layers, att, saved, dout, grads, *, heads, eps, drop, need_dx=True):
     """Backward of the whole stack (`hero_bert_stack_bwd`). grads: per layer a dict of fp32
-    tensors (keys of hero_layer_grads) that are ACCUMULATED into. Returns dx (bf16) or None.
-    `only_layer=l` differentiates just layer l (dout = gradient of that layer's output; the
-    result is the gradient of its input): the same native entry point on a one-layer slice.
-    `layer_events`: one torch.cuda.Event per layer, recorded where that layer's parameter
-    gradients are complete (`hero_stack_args.layer_done_events`)."""
+    tensors (keys of hero_layer_grads) that are ACCUMULATED into. Returns dx (bf16) or None."""
     _require_cuda(x, dout)
     assert dout.dtype == BF16 and dout.is_contiguous()
     ws, act_ptrs = saved
-    if only_layer is not None:
-        l = only_layer
-        if l > 0:   # the layer's input is the previous layer's saved output
-            M, H = x.shape
-            prev_out = act_ptrs[l - 1][_ACT_FIELDS.index("out")]
-            x = _PtrTensor(prev_out, (M, H), x.device)
-        layers, act_ptrs, grads = layers[l:l + 1], act_ptrs[l:l + 1], grads[l:l + 1]
     s, keep = _stack_struct(x, layers, att, heads, eps, drop, act_ptrs)
-    s.first_layer = only_layer or 0
     n = len(layers)
     G = (_lib.LayerGrads * n)()
     for i, gr in enumerate(grads):
@@ -390,10 +356,6 @@ def bert_stack_bwd(x, layers, att, saved, dout, grads, *, heads, eps, drop, need
     nbytes = _lib.lib().hero_bert_stack_bwd_scratch_bytes(s.n_tok, s.hidden, s.inter)
     scratch = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
     s.scratch = scratch.data_ptr()
-    if layer_events is not None:
-        assert len(layer_events) == n
-        evs = (C.c_void_p * n)(*[e.cuda_event for e in layer_events])
-        s.layer_done_events = evs
     _count(_STACK_BWD_LAUNCHES * n)
     _lib.check(_lib.lib().hero_bert_stack_bwd(C.byref(s), _stream()))
     return dx
@@ -462,16 +424,6 @@ def adamw_step(p, g, m, v, p_bf16, *, step_size, beta1, beta2, eps, lr_wd, grad_
     _lib.check(_lib.lib().hero_adamw_step(_ptr(p), _ptr(g), _ptr(m), _ptr(v), _ptr(p_bf16),
                                           p.numel(), step_size, beta1, beta2, eps, lr_wd,
                                           grad_scale, _ptr(clip_sumsq), clip_max_norm, _stream()))
-
-
-def reduce_slots(dst, slots, n_slots, slot_stride, scale, max_ctas=16):
-    """dst = (dst + sum of n_slots slices of `slots`, slot_stride apart) * scale, fp32, in place."""
-    _require_cuda(dst, slots)
-    assert dst.dtype == torch.float32 and slots.dtype == torch.float32 and dst.is_contiguous()
-    _count()
-    _lib.check(_lib.lib().hero_reduce_slots_f32(_ptr(dst), _ptr(slots), n_slots, slot_stride,
-                                                dst.numel(), scale, max_ctas, _stream()))
-    return dst
 
 
 def sumsq(x, out):

@@ -207,18 +207,6 @@ class FlatParams:
         return oa + na == ob
 
     # ------------------------------------------------------------------ flat gradients
-    def adopt_grad_buffer(self, buf):
-        """Use `buf` (fp32, >= total elements, e.g. symmetric memory shared with the peer GPUs) as
-        the flat gradient buffer; existing gradients are carried over."""
-        assert buf.dtype == torch.float32 and buf.numel() >= self.total and buf.is_contiguous()
-        new = buf[:self.total]
-        if self.grad_flat is not None:
-            new.copy_(self.grad_flat)
-        else:
-            new.zero_()
-        self.grad_flat = new
-        return self.ensure_flat_grads()
-
     def ensure_flat_grads(self):
         """Point every p.grad at a view of one flat fp32 buffer (absent grads are zeros), so the
         data-parallel all-reduce and the fused AdamW run on ONE tensor with no pack/unpack."""

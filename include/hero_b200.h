@@ -39,11 +39,6 @@ const char* hero_last_error(void);
 int hero_version(void);
 /* Returns SM count of the current device (148 on B200) or a negative hero_status. */
 int hero_sm_count(void);
-/* Size every persistent kernel for at most n SMs (0 = all). The GEMMs run one CTA per SM; while a
- * communication kernel (NCCL) holds some SMs a full-size grid would need a second wave for the
- * displaced CTAs. Used by hero_b200.distributed.GradBucketer(transport="nccl") while gradient
- * buckets are exchanged beside the backward kernels. */
-int hero_set_sm_limit(int32_t n);
 
 /* ------------------------------------------------------------------------------------------
  * GEMM family (tcgen05 / TMEM / TMA).   D[M,N] = epilogue( A · B^T-like contraction )
@@ -349,15 +344,6 @@ typedef struct hero_stack_args {
   const void* dout;              /* bf16 [n_tok, H] gradient of the last layer's output */
   void* dx;                      /* bf16 [n_tok, H] gradient of x (may be NULL for no input grad) */
   void* scratch;                 /* >= hero_bert_stack_bwd_scratch_bytes(...) bytes */
-  /* Index of weights[0] inside the full encoder (0 for a whole stack). Dropout masks are keyed by
-   * (drop_key, first_layer + l, site), so a caller may run the stack as several slices — e.g. one
-   * backward call per layer to overlap the gradient all-reduce — and get identical masks. */
-  int32_t first_layer;
-  /* Backward only, optional: n_layers CUDA events (cudaEvent_t). Event l is recorded at the point
-   * where every parameter gradient of layer l is complete (weight gradients run on the runtime's
-   * second stream), so a data-parallel caller can start exchanging layer l while the layers below
-   * are still being differentiated, from ONE call for the whole stack. */
-  void* const* layer_done_events;
 } hero_stack_args;
 
 int hero_bert_stack_fwd(const hero_stack_args* args, void* stream);
@@ -405,13 +391,6 @@ int hero_adamw_step(float* p, const float* g, float* m, float* v, void* p_bf16, 
 /* clip_sumsq != NULL folds global-norm clipping (train_vcmr.py:258-259) into the update without a
  * device->host round trip: g' is additionally scaled by min(1, clip_max_norm / (sqrt(*clip_sumsq)
  * + 1e-6)), *clip_sumsq being the device scalar accumulated by hero_sumsq_f32 over ALL gradients. */
-/* dst[i] = (dst[i] + sum_{s < n_slots} slots[s * slot_stride + i]) * scale, i < n (n, stride
- * multiples of 4), on at most max_ctas CTAs (0: 64). Reduction step of the copy-engine gradient
- * exchange (hero_b200.distributed.GradBucketer): peers deposit their slices of a bucket in `slots`
- * over NVLink with DMA copies; this is the only SM work of the exchange
- * (replaces the Horovod allreduce of utils/distributed.py:19-46 for the overlapped buckets). */
-int hero_reduce_slots_f32(float* dst, const float* slots, int32_t n_slots, int64_t slot_stride,
-                          int64_t n, float scale, int32_t max_ctas, void* stream);
 /* Combines the per-slab partials of an act-4 GEMM: lse[r] = log sum_c exp(v[r, c]) and
  * loss[r] = lse[r] - label_logit[r] (F.cross_entropy, reduction='none'), r < m. */
 int hero_ce_finish(const void* ce_partial, int64_t ld_partial, int32_t n_slabs,

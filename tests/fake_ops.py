@@ -278,14 +278,11 @@ def bert_stack_fwd(x, layers, att, *, heads, eps, drop, save, x_f32=None):
     return h, h32, (saved if save else None)
 
 
-def bert_stack_bwd(x, layers, att, saved, dout, grads, *, heads, eps, drop, need_dx=True,
-                   only_layer=None):
-    """Contract of `hero_bert_stack_bwd`: gradients are accumulated into `grads`; `only_layer`
-    differentiates a single layer (dout = gradient of that layer's output)."""
+def bert_stack_bwd(x, layers, att, saved, dout, grads, *, heads, eps, drop, need_dx=True):
+    """Contract of `hero_bert_stack_bwd`: gradients are accumulated into `grads`."""
     M, H = dout.shape
     dy = dout
-    order = range(len(layers) - 1, -1, -1) if only_layer is None else [only_layer]
-    for li in order:
+    for li in range(len(layers) - 1, -1, -1):
         lw, S, G = layers[li], saved[li], grads[li]
         inter = lw.w1.shape[0]
         ds2 = torch.empty(M, H, dtype=BF16)

@@ -4,6 +4,7 @@ of the reference (Horovod allreduce = mean over ranks; allgather concatenates in
 import os
 import socket
 
+import pytest
 import torch
 import torch.multiprocessing as mp
 
@@ -102,119 +103,9 @@ def test_single_process_degenerates_to_identity():
     assert hd.all_gather_list(7) == [7] and hd.any_broadcast("x", 0) == "x"
     x = torch.ones(2, 2, requires_grad=True)
     assert hd.vsm_allgather(x) is x or torch.equal(hd.vsm_allgather(x), x)
-
-
-class _Patch:
-    """monkeypatch stand-in for spawned workers (nothing to undo: the process exits)."""
-
-    @staticmethod
-    def setattr(obj, name, value):
-        setattr(obj, name, value)
-
-
-def _bucketer_case(rank, world, hd):
-    """Overlapped per-layer exchange == one all-reduce of the flat gradient after backward.
-    f_encoder is used twice per step (video-row subtitles and the query), so its layers may only be
-    exchanged after their second backward."""
-    import tempfile
-    from pathlib import Path
-    from tests import fake_ops, golden_util as gu
-    from tests.test_orchestration_cpu import _model
-    from hero_b200.params import flat_of
-    fake_ops.install(_Patch)
-    fx = gu.load("hier_tiny.npz")
-    vb, qb = gu.stored_batches(fx)
-    w1 = torch.from_numpy(fx["loss_w1"]) * (rank + 1)
-    w2 = torch.from_numpy(fx["loss_w2"]) * (2 - rank)
-
-    def loss_of(model):
-        clip = model(vb, "repr")
-        q = model.f_encoder(qb, "txt")[0]
-        return (clip * w1).sum() + (q * w2).sum()
-
-    out = []
-    with tempfile.TemporaryDirectory() as tmp:
-        for overlapped in (False, True):
-            model = _model(Path(tmp), fx)
-            flat = flat_of(model, torch.device("cpu"))
-            gflat = flat.ensure_flat_grads()
-            if overlapped:
-                bucketer = hd.GradBucketer(flat, min_elems=1)
-                with bucketer:
-                    loss_of(model).backward()
-                    early = len(bucketer.handles)
-                bucketer.finish(rescale_denom=2.0)
-                out.append(early)
-            else:
-                loss_of(model).backward()
-                hd.all_reduce_flat(gflat, 2.0)
-            out.append(gflat.clone())
-    return out
-
-
-def test_grad_bucketer_equals_single_allreduce():
-    res = _run("_bucketer_case")
-    for r in (0, 1):
-        plain, early, bucketed = res[r]
-        assert early >= 2                        # exchanges were issued during backward
-        assert torch.equal(plain, bucketed)
-    assert torch.equal(res[0][2], res[1][2])
-
-
-def test_peer_exchange_algorithm_on_simulated_ranks(monkeypatch):
-    """The copy-engine gradient exchange (distributed.PeerExchange: scatter into the owner's
-    staging slots -> reduce -> gather) run phase by phase over W simulated ranks that share this
-    process's memory: every rank must end with the mean of all ranks' buckets, for even, uneven and
-    tiny buckets, W = 2, 3, 8. (The CUDA pieces — symmetric memory, DMA copies, signals — are
-    exercised by tools/p2p_check.py on real GPUs.)"""
-    from hero_b200 import distributed as hd, ops
-
-    class Handle:                      # get_buffer(r, ...) = a view of rank r's tensor
-        def __init__(self, tensors):
-            self.tensors = tensors
-
-        def get_buffer(self, r, shape, dtype, offset):
-            return self.tensors[r][offset:offset + shape[0]]
-
-        def put_signal(self, r, ch):
-            pass
-
-        def wait_signal(self, r, ch):
-            pass
-
-    def reduce_slots(dst, slots, n_slots, stride, scale, max_ctas=16):
-        n = dst.numel()
-        acc = dst.clone()
-        for s in range(n_slots):
-            acc += slots[s * stride:s * stride + n]
-        dst.copy_(acc * scale)
-
-    monkeypatch.setattr(ops, "reduce_slots", reduce_slots)
-    total = 64 * 40
-    for W in (2, 3, 8):
-        gen = torch.Generator().manual_seed(W)
-        grads = [torch.randn(total + 64 * W, generator=gen) for _ in range(W)]
-        stages = [torch.full((total + 64 * W,), float("nan")) for _ in range(W)]
-        want = torch.stack(grads).mean(0)
-        ranks = []
-        for r in range(W):
-            ex = hd.PeerExchange.__new__(hd.PeerExchange)
-            ex.world, ex.rank, ex.grad, ex.stage, ex.channels = W, r, grads[r], stages[r], 16
-            ex.h_grad, ex.h_stage = Handle(grads), Handle(stages)
-            ranks.append(ex)
-        buckets = [(0, 64 * 16), (64 * 16, 64 * 17), (64 * 17, 64 * 39), (64 * 39, total)]
-        done = []
-        for a, b in buckets:
-            if not ranks[0].fits(a, b):
-                continue                       # GradBucketer sends such buckets through NCCL
-            done.append((a, b))
-            for phase in ("_scatter", "_reduce", "_gather"):
-                for ex in ranks:
-                    getattr(ex, phase)(a, b)
-        assert done, W
-        for a, b in done:
-            for r in range(W):
-                assert torch.allclose(grads[r][a:b], want[a:b], atol=1e-6), (W, a, b, r)
+    assert hd.overlapped_exchange(None, "none") is None
+    with pytest.raises(ValueError):
+        hd.overlapped_exchange(None, "p2p")
 
 
 def _vsm_scores_case(rank, world, hd):

@@ -190,60 +190,6 @@ def test_training_mode_dropout_runs_and_is_stochastic(tmp_path):
     assert g is not None and torch.isfinite(g).all() and g.abs().sum() > 0
 
 
-def test_per_layer_backward_with_grad_hook_matches_whole_stack(tmp_path):
-    """The data-parallel schedule (one native backward call per layer + GradBucketer hook) must
-    give the same gradients as the single whole-stack call — including the dropout masks, which
-    are keyed by the layer's index in the full encoder (hero_stack_args.first_layer). Same kernels
-    on the same data: the only difference allowed is the summation order of the split-K fp32
-    atomics of the weight gradients."""
-    from hero_b200 import functional
-    from hero_b200.params import flat_of
-    d = dict(hidden=768, inter=3072, heads=12, f_layers=3, c_layers=2, vocab=50272,
-             vfeat_dim=4352, max_img_len=100)
-    P = orc.seeded_weights(orc.param_shapes(f_layers=3, c_layers=2), seed=6)
-    vb, _ = synth.syn_tvr_ragged(batch_size=2, seed=4, t_range=(10, 20), s_range=(2, 4),
-                                 l_range=(4, 10))
-    vbd = synth.to_device(vb, "cuda")
-
-    class Hook:
-        def __init__(self, wants_events=False):
-            self.expected, self.ready_calls, self.events = 0, 0, 0
-            self.wants_events = wants_events
-
-        def expect(self, params):
-            self.expected += len(params)
-
-        def ready(self, params, event=None):
-            assert len(params) == 16
-            self.ready_calls += 1
-            if event is not None:
-                assert self.wants_events
-                event.synchronize()       # the layer's gradients are complete behind it
-                self.events += 1
-
-    grads = []
-    hooks = (None, Hook(), Hook(wants_events=True))
-    for hook in hooks:
-        model = _build(tmp_path, d, P).train()
-        gflat = flat_of(model, torch.device("cuda")).ensure_flat_grads()
-        functional.GRAD_HOOK[0] = hook
-        try:
-            torch.manual_seed(11)
-            out = model(vbd, "repr")
-            out.float().pow(2).mean().backward()
-        finally:
-            functional.GRAD_HOOK[0] = None
-        grads.append((out.detach().clone(), gflat.clone()))
-    for h in hooks[1:]:
-        assert h.ready_calls == 5 and h.expected == 16 * 5
-    assert hooks[1].events == 0 and hooks[2].events == 5   # one native call + one event per layer
-    a = grads[0][1]
-    assert a.abs().sum() > 0
-    for out, g in grads[1:]:
-        assert torch.equal(grads[0][0], out)
-        assert float((a - g).norm() / a.norm()) < 1e-5
-
-
 def test_hot_path_never_synchronises_with_collate_side_plans(tmp_path):
     """With plans attached on the host (collate / PlanPool) forward + backward must not contain a
     single device synchronisation — a hidden `.item()` / bool(tensor) drains the launch queue
