@@ -142,6 +142,9 @@ def _declare(lib):
     sig("hero_vsm_scores_bwd", vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp)
     sig("hero_vsm_span_fwd", vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp)
     sig("hero_vsm_span_bwd", vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp)
+    sig("hero_videoqa_pool_fwd", vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp)
+    sig("hero_videoqa_pool_bwd", vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp,
+        vp, vp)
 
 
 def lib():

@@ -9,6 +9,8 @@ gradients; the arithmetic reads the bf16 working copies held in `ctx_w` objects.
     cross_modal_embed   _compute_img_txt_embeddings   model/encoder.py:256-285 (+ embed.py:28-117)
     frame_merge         collect_frame_outputs + frame_transform residual  model/model.py:156-212
     frame_embed         FrameEmbeddings               model/embed.py:146-161
+    query_fused_embed   frame + QA embeddings of the video QA head    model/videoQA.py:68-79
+    videoqa_pool        HeroForVideoQA.get_modularized_video          model/videoQA.py:36-59
     pack / unpack       padded <-> packed layouts
 """
 import torch
@@ -419,6 +421,118 @@ class _FrameEmbed(torch.autograd.Function):
 
 def frame_embed(g, cfg, params):
     return _FrameEmbed.apply(g, cfg, *params)
+
+
+class _QueryFusedEmbed(torch.autograd.Function):
+    """Input of the video QA head's query-fused temporal stack (model/videoQA.py:68-79), written
+    straight into the packed joint rows (plan.VideoQaPlan): frame tokens
+    LN_c(g + c_pos[t]) (c_encoder.embeddings, the TemporalTrm frame embedding), QA tokens
+    LN_f(word[id] + f_pos[pid] + type[1]) (f_encoder.embeddings), each followed by dropout.
+    params: c_pos, c_ln_w, c_ln_b, word, f_pos, type, f_ln_w, f_ln_b. Returns the bf16 rows and
+    their fp32 copy (residual of the first layer).
+    The backward does not signal EXCHANGE_HOOK: the cross-modal embedding backward that runs after
+    it is the last node of the graph, and the QA gradients land in f_encoder.embeddings, whose
+    range is exchanged after that node anyway (params.LATE_GRAD)."""
+
+    @staticmethod
+    def forward(ctx, g, cfg, c_pos, c_ln_w, c_ln_b, word, f_pos, typ, f_ln_w, f_ln_b):
+        drop = cfg["drop"]
+        dev = g.device
+        H = g.shape[1]
+        n_c, n_qa = cfg["n_frame"], cfg["n_qa"]
+        emb = torch.empty((cfg["n_tok"], H), dtype=BF16, device=dev)
+        emb32 = torch.empty((cfg["n_tok"], H), dtype=F32, device=dev)
+        st = {}
+        st["f_mean"], st["f_rstd"] = torch.empty(n_c, device=dev), torch.empty(n_c, device=dev)
+        st["f_drop"] = drop.next(drop.hidden_p)
+        ops.ln_fwd(g, c_ln_w, c_ln_b, 1e-5, emb, n_rows=n_c, add_tab=c_pos, add_idx=cfg["c_t"],
+                   y_rows=cfg["c_row"], mean=st["f_mean"], rstd=st["f_rstd"], drop=st["f_drop"],
+                   y_f32=emb32)
+        if n_qa:
+            st["q_mean"] = torch.empty(n_qa, device=dev)
+            st["q_rstd"] = torch.empty(n_qa, device=dev)
+            st["q_drop"] = drop.next(drop.hidden_p)
+            ops.ln_fwd(word, f_ln_w, f_ln_b, 1e-5, emb, n_rows=n_qa, x_rows=cfg["qa_ids"],
+                       add_tab=f_pos, add_idx=cfg["qa_pos"], add_vec=typ[1], y_rows=cfg["qa_row"],
+                       mean=st["q_mean"], rstd=st["q_rstd"], drop=st["q_drop"], y_f32=emb32)
+        ctx.cfg, ctx.st = cfg, st
+        ctx.save_for_backward(g)
+        ctx.params = (c_pos, c_ln_w, c_ln_b, word, f_pos, typ, f_ln_w, f_ln_b)
+        ctx.mark_non_differentiable(emb32)
+        return emb, emb32
+
+    @staticmethod
+    def backward(ctx, demb, _demb32=None):
+        cfg, st = ctx.cfg, ctx.st
+        (g,) = ctx.saved_tensors
+        c_pos, c_ln_w, c_ln_b, word, f_pos, typ, f_ln_w, f_ln_b = ctx.params
+        demb = demb.contiguous()
+        n_c, n_qa = cfg["n_frame"], cfg["n_qa"]
+        grads = [None] * 8
+        dg = torch.empty_like(g)
+        dclnw, grads[1] = _sink(c_ln_w)
+        dclnb, grads[2] = _sink(c_ln_b)
+        ops.ln_bwd(demb, g, c_ln_w, st["f_mean"], st["f_rstd"], n_rows=n_c, add_tab=c_pos,
+                   add_idx=cfg["c_t"], y_rows=cfg["c_row"], drop=st["f_drop"], dx=dg,
+                   dgamma=dclnw, dbeta=dclnb)
+        dcpos, grads[0] = _sink(c_pos)
+        ops.gather_sum_rows(dg, cfg["c_pos_off"], cfg["c_pos_idx"],
+                            dcpos[:cfg["c_pos_off"].numel() - 1])
+        if n_qa:
+            dword, grads[3] = _sink(word)
+            dfpos, grads[4] = _sink(f_pos)
+            dtyp, grads[5] = _sink(typ)
+            dflnw, grads[6] = _sink(f_ln_w)
+            dflnb, grads[7] = _sink(f_ln_b)
+            dq = torch.empty((n_qa, g.shape[1]), dtype=BF16, device=g.device)
+            # the word-table scatter-add skips the padding id, as _CrossModalEmbed does
+            ops.ln_bwd(demb, word, f_ln_w, st["q_mean"], st["q_rstd"], n_rows=n_qa,
+                       x_rows=cfg["qa_ids"], add_tab=f_pos, add_idx=cfg["qa_pos"],
+                       add_vec=typ[1], y_rows=cfg["qa_row"], drop=st["q_drop"], dx=dq,
+                       d_x_tab=dword, x_pad_idx=cfg["pad_idx"], dgamma=dflnw, dbeta=dflnb)
+            ops.gather_sum_rows(dq, cfg["qa_pos_off"], cfg["qa_pos_idx"],
+                                dfpos[:cfg["qa_pos_off"].numel() - 1])
+            ops.colsum(dq, dtyp[1])
+        ctx.st = None
+        return (dg, None) + tuple(grads)
+
+
+def query_fused_embed(g, cfg, params):
+    return _QueryFusedEmbed.apply(g, cfg, *params)
+
+
+class _VideoQaPool(torch.autograd.Function):
+    """(P_se [Nv, T, H], P_qa [Nv, Nq, H]) = modularized-video pooling of the frame rows of the
+    packed fp32 stack output y (model/videoQA.py:36-59; hero_b200/csrc/videoqa.cu). The gradient
+    of y is zero at the QA-token rows, which the reference slices off (model/videoQA.py:82)."""
+
+    @staticmethod
+    def forward(ctx, y, frame_tok, w_se, w_qa, nv, nq, t):
+        y = y.contiguous()
+        ws, wq = w_se.detach().reshape(-1), w_qa.detach().reshape(-1)
+        p_se, p_qa, a_se, a_qa = ops.videoqa_pool_fwd(y, frame_tok, ws, wq, nv, nq, t)
+        ctx.st = (y, frame_tok, ws, wq, a_se, a_qa, (nv, nq, t))
+        ctx.params = (w_se, w_qa)
+        return p_se, p_qa
+
+    @staticmethod
+    def backward(ctx, dp_se, dp_qa):
+        y, frame_tok, ws, wq, a_se, a_qa, (nv, nq, t) = ctx.st
+        w_se, w_qa = ctx.params
+        H = y.shape[1]
+        dp_se = _zeros((nv, t, H), y) if dp_se is None else dp_se.float().contiguous()
+        dp_qa = _zeros((nv, nq, H), y) if dp_qa is None else dp_qa.float().contiguous()
+        dy = torch.zeros_like(y)
+        dws, r_se = _sink(w_se)
+        dwq, r_qa = _sink(w_qa)
+        ops.videoqa_pool_bwd(y, frame_tok, ws, wq, a_se, a_qa, dp_se, dp_qa, nv, nq, t, dy,
+                             dws.view(-1), dwq.view(-1))
+        ctx.st = None
+        return dy, None, r_se, r_qa, None, None, None
+
+
+def videoqa_pool(y, frame_tok, w_se, w_qa, nv, nq, t):
+    return _VideoQaPool.apply(y, frame_tok, w_se, w_qa, nv, nq, t)
 
 
 # ---------------------------------------------------------------------------------------------

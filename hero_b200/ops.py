@@ -489,6 +489,42 @@ def vsm_span_bwd(dst, ded, mask_u8, w_st, w_ed, sim, query, ctx, dquery, dctx, d
 
 
 # ---------------------------------------------------------------------------------------------
+# Video QA head (hero_b200/csrc/videoqa.cu)
+def videoqa_pool_fwd(y, frame_tok, w_se, w_qa, nv, nq, t):
+    """Modularized-video pooling (model/videoQA.py:36-59) over the frame rows of the packed fp32
+    stack output y [n_joint, H]. Returns (p_se [nv, t, H], p_qa [nv, nq, H], a_se, a_qa), the a_*
+    being the two softmax probability tensors [nv, nq, t] the backward needs."""
+    _require_cuda(y, frame_tok, w_se, w_qa)
+    for x in (y, w_se, w_qa):
+        assert x.dtype == torch.float32 and x.is_contiguous()
+    assert frame_tok.dtype == torch.int32 and frame_tok.numel() == nv * nq * t
+    h = y.shape[1]
+    s = torch.empty((4, nv, nq, t), dtype=torch.float32, device=y.device)
+    p_se = torch.empty((nv, t, h), dtype=torch.float32, device=y.device)
+    p_qa = torch.empty((nv, nq, h), dtype=torch.float32, device=y.device)
+    _count(2)
+    _lib.check(_lib.lib().hero_videoqa_pool_fwd(_ptr(y), _ptr(frame_tok), _ptr(w_se), _ptr(w_qa),
+                                                nv, nq, t, h, _ptr(s[0]), _ptr(s[1]), _ptr(s[2]),
+                                                _ptr(s[3]), _ptr(p_se), _ptr(p_qa), _stream()))
+    return p_se, p_qa, s[2], s[3]
+
+
+def videoqa_pool_bwd(y, frame_tok, w_se, w_qa, a_se, a_qa, dp_se, dp_qa, nv, nq, t, dy, dw_se,
+                     dw_qa):
+    """dy (fp32 [n_joint, H]) is OVERWRITTEN at the frame rows only; dw_se / dw_qa (fp32 [H]) are
+    accumulated."""
+    _require_cuda(y, frame_tok, dp_se, dp_qa, dy, dw_se, dw_qa)
+    for x in (y, w_se, w_qa, a_se, a_qa, dp_se, dp_qa, dy, dw_se, dw_qa):
+        assert x.dtype == torch.float32 and x.is_contiguous()
+    da = torch.empty((2, nv, nq, t), dtype=torch.float32, device=y.device)
+    _count(2)
+    _lib.check(_lib.lib().hero_videoqa_pool_bwd(_ptr(y), _ptr(frame_tok), _ptr(w_se), _ptr(w_qa),
+                                                _ptr(a_se), _ptr(a_qa), _ptr(dp_se), _ptr(dp_qa),
+                                                nv, nq, t, y.shape[1], _ptr(da[0]), _ptr(da[1]),
+                                                _ptr(dy), _ptr(dw_se), _ptr(dw_qa), _stream()))
+
+
+# ---------------------------------------------------------------------------------------------
 # Fused LM-head cross entropy (MLM): vocabulary logits are never materialised in fp32.
 def lm_head_ce_fwd(h, emb, bias, labels, n_valid):
     """h: bf16 [n, H] (LM-head transform of the masked tokens), emb: bf16 [V, H] (tied word

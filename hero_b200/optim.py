@@ -5,19 +5,21 @@ the un-corrected lr, no decay for names containing 'bias' / 'LayerNorm.*'.
 
 The reference launches ~10 pointwise kernels for each of ~208 tensors per step; here the flat
 layout (decayed parameters first, see params.py) needs TWO launches, and the same kernel refreshes
-the bf16 working copy so the next forward skips its cast pass.
+the bf16 working copy so the next forward skips its cast pass. With `lr_mul != 1` (the fine-tuning
+heads, e.g. train_videoQA.py) the reference's four groups are kept: each is a short list of
+contiguous flat ranges, one launch per range.
 """
 import math
 
 import torch
 
 from . import ops
-from .params import FlatParams
+from .params import FlatParams, is_no_decay
 
 
 class FusedAdamW:
     def __init__(self, flat, lr=1e-4, betas=(0.9, 0.98), eps=1e-6, weight_decay=0.01,
-                 correct_bias=True):
+                 correct_bias=True, lr_mul=1.0):
         assert isinstance(flat, FlatParams) and flat.flat is not None, \
             "call flat_of(model, device) (or run one forward) before building the optimizer"
         self.flat = flat
@@ -26,12 +28,23 @@ class FusedAdamW:
         self.eps = eps
         self.betas = betas
         split = flat.no_decay_start
-        # `param_groups` keeps the reference loop working:
+        # `param_groups` keeps the reference loops working:
         #     for g in optimizer.param_groups: g['lr'] = lr_this_step   (train_vcmr.py:245-247)
-        self.param_groups = [
-            {"lr": lr, "weight_decay": weight_decay, "range": (0, split)},
-            {"lr": lr, "weight_decay": 0.0, "range": (split, flat.total)},
-        ]
+        #     param_groups[0, 1]['lr'] = lr * lr_mul; [2, 3]['lr'] = lr (train_videoQA.py:186-192)
+        if float(lr_mul) == 1.0:
+            self.param_groups = [
+                {"lr": lr, "weight_decay": weight_decay, "ranges": [(0, split)]},
+                {"lr": lr, "weight_decay": 0.0, "ranges": [(split, flat.total)]},
+            ]
+        else:
+            self.param_groups = [
+                {"lr": lr * lr_mul, "weight_decay": weight_decay, "ranges": []},
+                {"lr": lr * lr_mul, "weight_decay": 0.0, "ranges": []},
+                {"lr": lr, "weight_decay": weight_decay, "ranges": []},
+                {"lr": lr, "weight_decay": 0.0, "ranges": []},
+            ]
+            for grp, a, b in _group_ranges(flat):
+                self.param_groups[grp]["ranges"].append((a, b))
         self.exp_avg = torch.zeros_like(flat.flat)
         self.exp_avg_sq = torch.zeros_like(flat.flat)
         self.step_count = 0
@@ -79,18 +92,19 @@ class FusedAdamW:
         clip = getattr(self, "_clip", None)
         self._clip = None
         for grp in self.param_groups:
-            a, b = grp["range"]
-            if b <= a:
-                continue
             lr = grp["lr"]
             step_size = lr
             if self.correct_bias:
                 step_size = lr * math.sqrt(1.0 - b2 ** t) / (1.0 - b1 ** t)
-            ops.adamw_step(self.flat.flat[a:b], g[a:b], self.exp_avg[a:b], self.exp_avg_sq[a:b],
-                           self.flat.mirror[a:b], step_size=step_size, beta1=b1, beta2=b2,
-                           eps=self.eps, lr_wd=lr * grp["weight_decay"], grad_scale=scale,
-                           clip_sumsq=self._sumsq if clip is not None else None,
-                           clip_max_norm=clip or 0.0)
+            for a, b in grp["ranges"]:
+                if b <= a:
+                    continue
+                ops.adamw_step(self.flat.flat[a:b], g[a:b], self.exp_avg[a:b],
+                               self.exp_avg_sq[a:b], self.flat.mirror[a:b], step_size=step_size,
+                               beta1=b1, beta2=b2, eps=self.eps, lr_wd=lr * grp["weight_decay"],
+                               grad_scale=scale,
+                               clip_sumsq=self._sumsq if clip is not None else None,
+                               clip_max_norm=clip or 0.0)
         # masters changed in place through a flat view: the mirror is already fresh
         self.flat.dirty = False
         self.flat._version_sum = sum(p._version for _, p, _, _ in self.flat._probe)
@@ -107,19 +121,31 @@ class FusedAdamW:
             g["lr"], g["weight_decay"] = s["lr"], s["weight_decay"]
 
 
+def _group_ranges(flat):
+    """(group, start, end) per maximal run of flat entries in one of the reference's four groups
+    (optim/misc.py:14-37): 0 top-level decay, 1 top-level no-decay, 2 v_encoder decay,
+    3 v_encoder no-decay. A run reaches to the next entry's offset (alignment padding included)."""
+    runs = []
+    ends = [off for _, _, off, _ in flat.entries[1:]] + [flat.total]
+    for (name, _, off, _), end in zip(flat.entries, ends):
+        grp = 2 * ("v_encoder" in name) + is_no_decay(name)
+        if runs and runs[-1][0] == grp and runs[-1][2] == off:
+            runs[-1][2] = end
+        else:
+            runs.append([grp, off, end])
+    return [tuple(r) for r in runs]
+
+
 def build_optimizer(model, opts, device=None):
-    """optim/misc.py:14-50 for optim == 'adamw' on the flat layout. The reference builds FOUR
-    groups (top x lr_mul decay / no-decay, v_encoder decay / no-decay) and some of its loops index
-    them (`if i in (0, 1): lr *= lr_mul`, train_videoQA.py); the flat layout has TWO ranges
-    (decay, no-decay), so anything that would make the four groups differ is refused instead of
-    being silently collapsed: lr_mul != 1, optimizers other than AdamW, frozen parameters."""
+    """optim/misc.py:14-50 for optim == 'adamw' on the flat layout. With lr_mul == 1 the
+    reference's four groups share one learning rate and collapse to TWO flat ranges (decay,
+    no-decay). With lr_mul != 1 `param_groups` are the reference's four groups in its order (top
+    level x lr_mul decay / no-decay, v_encoder decay / no-decay), which its fine-tuning loops index
+    (train_videoQA.py:186-192). Refused: optimizers other than AdamW, frozen parameters."""
     from .params import flat_of
     if getattr(opts, "optim", "adamw") != "adamw":
         raise ValueError(f"hero_b200.build_optimizer implements 'adamw' only (got {opts.optim!r}); "
                          "use the reference's torch optimizer for adam / adamax")
-    if float(getattr(opts, "lr_mul", 1.0)) != 1.0:
-        raise ValueError("lr_mul != 1 needs the reference's four parameter groups; FusedAdamW "
-                         "keeps two flat ranges (decay / no-decay) with one learning rate")
     frozen = [n for n, p in model.named_parameters() if not p.requires_grad]
     if frozen:
         raise ValueError(f"frozen parameters ({frozen[:3]}...) are not supported by the flat "
@@ -127,4 +153,4 @@ def build_optimizer(model, opts, device=None):
     device = device or next(model.parameters()).device
     flat = flat_of(model, device)
     return FusedAdamW(flat, lr=opts.learning_rate, betas=tuple(opts.betas),
-                      weight_decay=opts.weight_decay)
+                      weight_decay=opts.weight_decay, lr_mul=float(getattr(opts, "lr_mul", 1.0)))

@@ -414,6 +414,65 @@ class JointPlan:
                 "n_tok": self.n_tok, "n_seq": self.n_seq, "max_len": self.max_len}
 
 
+class VideoQaPlan:
+    """Query-fused temporal stage of the video QA head (model/videoQA.py:66-82): per (question,
+    answer candidate) row r = v * Nq + q the joint sequence is the row's valid clip frames followed
+    by its valid QA tokens, i.e. a SeqPlan over cat(c_attn_masks, qa_attn_masks, dim=1) (row-major
+    packing). Rows over 128 tokens (T = 100 frames + 30 QA tokens) take SeqPlan's long-sequence
+    tiles.
+        c_row     per clip token (CPlan order): its joint row (scatter target of the frame half)
+        qa_row    per QA token: its joint row; qa_ids / qa_pos: its vocabulary / position id
+        frame_tok [Nv, Nq, T]: joint row of frame t of candidate q of question v, -1 if padded
+    `cplan` is the CPlan of the same batch (ReprPlan.c)."""
+
+    def __init__(self, c_attn_masks, qa_attn_masks, qa_input_ids, qa_pos_ids, n_questions, cplan):
+        cm, qm = _np(c_attn_masks) != 0, _np(qa_attn_masks) != 0
+        rows, T = cm.shape
+        L = qm.shape[1]
+        if qm.shape[0] != rows:
+            raise ValueError(f"{qm.shape[0]} QA rows for {rows} clip rows")
+        self.nv = int(n_questions)
+        if self.nv <= 0 or rows % self.nv:
+            raise ValueError(f"{rows} (question, answer) rows are not a multiple of {self.nv} "
+                             "questions")
+        self.nq, self.t = rows // self.nv, T
+        self.seq = SeqPlan(np.concatenate([cm, qm], axis=1))
+        W = T + L
+        p2t = self.seq.pad_to_tok
+        self.c_row = p2t[cplan.seq.tok_row.astype(np.int64) * W + cplan.seq.tok_col]
+        qr, qc = np.nonzero(qm)
+        self.qa_row = p2t[qr.astype(np.int64) * W + T + qc]
+        self.n_qa = int(qr.size)
+        self.n_frame = int(self.c_row.size)
+        ids = np.asarray(_np(qa_input_ids), np.int64)     # device tensors: read back (one sync)
+        pos = np.asarray(_np(qa_pos_ids), np.int64).reshape(-1, L)
+        self.qa_ids = ids[qr, qc].astype(np.int32)
+        self.qa_pos = (pos[0][qc] if pos.shape[0] == 1 else pos[qr, qc]).astype(np.int32)
+        # position-table CSR over ids 0 .. max id (deterministic table gradient)
+        self.n_pos = int(self.qa_pos.max()) + 1 if self.n_qa else 1
+        self.qa_pos_off, self.qa_pos_idx = table_csr(self.qa_pos, self.n_pos)
+        self.frame_tok = np.where(cm, p2t.reshape(rows, W)[:, :T], -1).astype(np.int32)
+        self.dev = None
+
+    def to(self, device, staging=None):
+        device = torch.device(device)
+        if self.dev is None or self.dev.flat.device != device:
+            a = self.seq.arrays("j_")
+            a.update({"c_row": self.c_row, "qa_row": self.qa_row, "qa_ids": self.qa_ids,
+                      "qa_pos": self.qa_pos, "qa_pos_off": self.qa_pos_off,
+                      "qa_pos_idx": self.qa_pos_idx, "frame_tok": self.frame_tok})
+            self.dev = DeviceIndex(a, device, staging)
+        return self.dev
+
+
+def videoqa_plans(batch):
+    """(ReprPlan, VideoQaPlan) of a video QA batch (data/videoQA.py video_qa_collate layout)."""
+    rplan = ReprPlan(batch)
+    vplan = VideoQaPlan(batch["c_attn_masks"], batch["qa_attn_masks"], batch["qa_input_ids"],
+                        batch["qa_pos_ids"], len(batch["targets"]), rplan.c)
+    return rplan, vplan
+
+
 PLAN_KEY = "_hero_plan"
 _REPR_KEYS = ("f_attn_masks", "f_gather_index", "c_attn_masks", "num_subs", "sub_idx2frame_idx")
 
@@ -477,6 +536,7 @@ class PlanPool:
 
 
 QUERY_PLAN_KEY = "_hero_query_plan"
+VIDEOQA_PLAN_KEY = "_hero_videoqa_plan"
 
 
 def attach_plan(batch, kind="repr"):
@@ -484,7 +544,9 @@ def attach_plan(batch, kind="repr"):
     the batch dict; `move_to_cuda`-style helpers leave non-tensor values alone.
     kind: 'repr' (video batch), 'txt' (query batch), or 'vsm' — a VSM / VCMR training batch that
     carries its queries as `query_input_ids / query_pos_ids / query_attn_masks` (data/vcmr.py):
-    attaches the video plan, the query plan (QUERY_PLAN_KEY) and their joint plan.
+    attaches the video plan, the query plan (QUERY_PLAN_KEY) and their joint plan; or 'videoqa'
+    — a TVQA / How2QA batch (data/videoQA.py): the video plan and the query-fused temporal plan
+    (VIDEOQA_PLAN_KEY, see VideoQaPlan).
     The plan captures the batch's token / position ids per packed token (FPlan.gather_ids): attach
     it AFTER any masking of `input_ids` (the reference masks in the dataset, before collate), and
     attach again if the ids are edited afterwards."""
@@ -494,6 +556,9 @@ def attach_plan(batch, kind="repr"):
                         input_ids=batch.get("query_input_ids"))
         rplan.__dict__["_joint"] = JointPlan(rplan, tplan)
         batch[PLAN_KEY], batch[QUERY_PLAN_KEY] = rplan, tplan
+        return batch
+    if kind == "videoqa":
+        batch[PLAN_KEY], batch[VIDEOQA_PLAN_KEY] = videoqa_plans(batch)
         return batch
     if kind == "repr":
         batch[PLAN_KEY] = ReprPlan(batch)

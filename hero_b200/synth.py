@@ -257,3 +257,63 @@ def syn_vsm_batch(vb, qb, seed=0):
     b.update(query_input_ids=qb["input_ids"], query_pos_ids=qb["pos_ids"],
              query_attn_masks=qb["attn_masks"], targets=torch.tensor(tg, dtype=torch.long))
     return b
+
+
+# --------------------------------------------------------------------------------------------
+# Video QA (TVQA / How2QA): data/videoQA.py. Every (question, answer candidate) pair becomes one
+# clip row whose subtitles carry the QA text appended ([SEP] question [SEP] answer,
+# data/videoQA.py:93-109); the QA text alone is collated as `qa_*` (txt_input_collate).
+def make_qa_question(gen, clip, qa_lens, target, ts, vocab=50265):
+    """One question: the clip item, one QA token row per answer candidate, the answer index and
+    the (start, end) frame target (-1 entries are ignored by the losses)."""
+    qas = []
+    for L in qa_lens:
+        ids = torch.randint(3, vocab, (L,), generator=gen)
+        ids[0] = SEP
+        ids[L // 3] = SEP
+        qas.append(ids)
+    return {"clip": clip, "qas": qas, "target": int(target), "ts": (int(ts[0]), int(ts[1]))}
+
+
+def videoqa_batch(questions):
+    """Collate questions into the batch dict of data/videoQA.py video_qa_collate."""
+    clips, qa_ids = [], []
+    for qn in questions:
+        c = qn["clip"]
+        for qa in qn["qas"]:
+            clips.append({"feats": c["feats"], "sub2frames": c["sub2frames"],
+                          "subs": [torch.cat([s, qa]) for s in c["subs"]]})
+            qa_ids.append(qa)
+    batch = video_batch(clips)
+    n, max_l = len(qa_ids), max(len(q) for q in qa_ids)
+    ids = torch.full((n, max_l), PAD, dtype=torch.long)
+    masks = torch.zeros(n, max_l, dtype=torch.long)
+    for i, q in enumerate(qa_ids):
+        ids[i, :len(q)] = q
+        masks[i, :len(q)] = 1
+    batch["targets"] = torch.tensor([[qn["target"]] for qn in questions], dtype=torch.long)
+    batch["ts_targets"] = torch.tensor([list(qn["ts"]) for qn in questions], dtype=torch.long)
+    batch["qa_input_ids"] = ids
+    batch["qa_pos_ids"] = torch.arange(max_l, dtype=torch.long).clamp(max=511).unsqueeze(0)
+    batch["qa_attn_masks"] = masks
+    return batch
+
+
+def syn_tvqa(n_questions=4, n_cand=5, n_frames=60, seed=3456, n_subs=12, frames_per_sub=5,
+             sub_len=14, qa_len=30, vfeat_dim=VFEAT_DIM, vocab=50265):
+    """SYN-TVQA: 4 questions x 5 candidates, T = 60, 12 subtitles of 5 frames + 14 tokens, 30 QA
+    tokens (49-token cross-modal rows, 90-token joint rows). n_frames=100 gives SYN-TVQA-long:
+    130-token joint rows, all on the long-sequence attention tiles. Shapes chosen to cover both
+    attention paths, not dataset statistics."""
+    gen = torch.Generator().manual_seed(seed)
+    rnd = random.Random(seed)
+    questions = []
+    for _ in range(n_questions):
+        frames = [range(s * frames_per_sub, min((s + 1) * frames_per_sub, n_frames))
+                  for s in range(n_subs)]
+        clip = make_clip(gen, n_frames, frames, [sub_len] * n_subs, vfeat_dim, vocab)
+        st = rnd.randrange(0, n_frames - 1)
+        ed = min(n_frames - 1, st + rnd.randrange(1, 10))
+        questions.append(make_qa_question(gen, clip, [qa_len] * n_cand,
+                                          rnd.randrange(n_cand), (st, ed), vocab))
+    return videoqa_batch(questions)

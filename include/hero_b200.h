@@ -434,6 +434,30 @@ int hero_vsm_span_bwd(const float* dst, const float* ded, const uint8_t* mask, c
                       int32_t n, int32_t len, int32_t d, int32_t k, float* dquery, float* dctx,
                       float* dw_st, float* dw_ed, void* stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Video question answering head (TVQA / How2QA): HeroForVideoQA.get_modularized_video,
+ * model/videoQA.py:36-59, on the packed fp32 output y [n_joint, h] of the query-fused temporal
+ * stack (model/videoQA.py:66-82). frame_tok [nv * nq * t] is the row of y holding frame t of
+ * answer candidate q of question v, or -1 at a padded frame (x = 0 there). With x = y[frame_tok]:
+ *   s_se = w_se . x, s_qa = w_qa . x; score where valid, exactly -1e4 where not (mask_logits)
+ *   a_se = softmax over q (videoQA.py:45-47), a_qa = softmax over t (videoQA.py:48-50)
+ *   p_se [nv, t, h] = sum_q a_se x (videoQA.py:52-54), p_qa [nv, nq, h] = sum_t a_qa x (:55-57)
+ * s_se / s_qa / a_se / a_qa are [nv, nq, t] fp32 (the a_* feed the backward). nq <= 64,
+ * t <= 1024, h % 4 == 0. Two kernel launches. */
+int hero_videoqa_pool_fwd(const float* y, const int32_t* frame_tok, const float* w_se,
+                          const float* w_qa, int32_t nv, int32_t nq, int32_t t, int32_t h,
+                          float* s_se, float* s_qa, float* a_se, float* a_qa, float* p_se,
+                          float* p_qa, void* stream);
+/* Backward given dp_se / dp_qa: dy [n_joint, h] receives d loss / dx at every frame row
+ * (OVERWRITTEN there; other rows, the QA tokens sliced off at model/videoQA.py:82, are not
+ * touched: zero them first); dw_se / dw_qa [h] are ACCUMULATED (+=). The softmax Jacobian terms
+ * are zero at padded frames. da_se / da_qa: [nv, nq, t] fp32 scratch. Two kernel launches. */
+int hero_videoqa_pool_bwd(const float* y, const int32_t* frame_tok, const float* w_se,
+                          const float* w_qa, const float* a_se, const float* a_qa,
+                          const float* dp_se, const float* dp_qa, int32_t nv, int32_t nq,
+                          int32_t t, int32_t h, float* da_se, float* da_qa, float* dy,
+                          float* dw_se, float* dw_qa, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
